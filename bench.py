@@ -2,7 +2,7 @@
 """bench.py -- the decoding hot path on N B200s: one JSON line with throughput, roofline, end-to-end and CPU-baseline
 figures for one workload.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--no-extras]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--workload NAME] [--impl reference] [--no-extras] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N --master-addr 127.0.0.1 --master-port P \
         bench.py --gpus N --steps K --warmup W [--workload NAME]
 
@@ -22,6 +22,11 @@ point -- are split: strong).  `e2e` times the same
 work through the public host-buffer API (pinned host memory, H2D and D2H inside the timed region).
 `--impl reference` times the CPU restatement of the reference's algorithm (oracle/, fp64, all host threads) on the same
 workload -- the Python reference itself cannot travel to the GPU box (BASELINE.md section 2: ~1.5 codewords/s/core).
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step computed as DIR/<name>.npy (float32 / float64,
+<= 64 MB in all): the decoded bits (of a fixed seeded sample of frames where they are larger), the LDPC iteration counts or
+the link's BER per point, and the step's error counters.  The inputs depend on the arguments only, so two builds run with
+the same arguments can be compared output for output.  Keeping the sample is part of the last timed step (Viterbi: one
+gather per launch), so time without the flag.
 """
 import argparse
 import json
@@ -174,20 +179,30 @@ def count_errors(dec, msg, counters, torch):
     _lib.check(rc, "count_errors")
 
 
+def dump_rows(n, k):
+    """the frames --dump-outputs writes of an output too large to write whole: k of n, a fixed seeded sample, sorted"""
+    return np.sort(np.random.RandomState(0).choice(n, min(n, k), replace=False))
+
+
 # ------------------------------------------------------------------------------------------------ workloads
 class Workload:
     """One BASELINE config.  Subclasses fill in: describe() (IDENTICAL in both arms), make(), step(), units, roofline data,
-    e2e_*(), parity(), cpu_sample()."""
+    e2e_*(), parity(), cpu_sample(), outputs()."""
     metric = HEADLINE_METRIC
     unit = "codewords/s"
     scaling = "weak"
     ncounters = 2
+    capture = False             # set for the last timed step under --dump-outputs: step() then keeps what it computed
 
     def units_per_step(self, world):           # whole-job units processed by one step on `world` ranks
         raise NotImplementedError
 
     def finish(self, counters):
         return {}
+
+    def outputs(self, torch):
+        """what the captured step handed its caller, as float32 / float64 numpy arrays by name"""
+        raise NotImplementedError
 
 
 class ViterbiWorkload(Workload):
@@ -252,17 +267,27 @@ class ViterbiWorkload(Workload):
             self.msgs.append(msg)
             del coded, pad
         self.out = torch.empty((self.batch, self.nbits), dtype=torch.uint8, device="cuda")
+        self.dump_idx = torch.from_numpy(dump_rows(self.batch, 512)).cuda()
         self.kernel_launches_per_step = self.launches * (2 if self.mode == "hard" else 3)   # decode [+ frame scale] + count
 
     def step(self, torch, counters, ev=None):
         from commpy_b200.channelcoding import viterbi_decode_batch
+        kept = [] if self.capture else None
         for i in range(self.launches):
             if ev is not None and i == 0:
                 ev[0].record()
             viterbi_decode_batch(self.inputs[i], self.trellis, None, self.mode, out=self.out)
             if ev is not None and i == 0:
                 ev[1].record()
+            if kept is not None:                 # every launch overwrites self.out: keep the sampled frames of each
+                kept.append(self.out.index_select(0, self.dump_idx))
             count_errors(self.out, self.msgs[i], counters, torch)
+        if kept is not None:
+            self.kept = kept
+
+    def outputs(self, torch):
+        """decoded bits of the same 512 sampled frames of every launch: (launches, 512, nbits)"""
+        return {"decoded_bits": torch.stack(self.kept).float().cpu().numpy()}
 
     def kernel_units(self):                      # units the event-timed launch processes
         return self.batch
@@ -402,6 +427,13 @@ class TurboWorkload(Workload):
         if ev is not None:
             ev[1].record()
         count_errors(bits, self.zero, counters, torch)
+        if self.capture:
+            self.last_bits = bits
+
+    def outputs(self, torch):
+        """decoded bits of 1,024 sampled codewords of this rank: (1024, N)"""
+        rows = torch.from_numpy(dump_rows(self.batch, 1024)).cuda()
+        return {"decoded_bits": self.last_bits.index_select(0, rows).float().cpu().numpy()}
 
     def kernel_units(self):
         return self.batch
@@ -494,6 +526,12 @@ class LdpcWorkload(Workload):
             ev[1].record()
         self.last_it = it
         count_errors(dec, self.zero, counters, torch)
+        if self.capture:
+            self.last_dec = dec
+
+    def outputs(self, torch):
+        """hard decisions of every frame (batch, n) and the iterations each frame ran (batch,)"""
+        return {"decoded_bits": self.last_dec.float().cpu().numpy(), "iterations": self.last_it.float().cpu().numpy()}
 
     def kernel_units(self):
         return self.batch
@@ -589,6 +627,10 @@ class LinkWorkload(Workload):
         if ev is not None:
             ev[1].record()
         counters += tot
+
+    def outputs(self, torch):
+        """BER of every point of the sweep"""
+        return {"ber_per_point": np.asarray(self.bers, dtype=np.float64)}
 
     def kernel_units(self):
         return self.units_per_step(1)
@@ -758,6 +800,9 @@ def run_b200(args):
     barrier()
     e0.record()
     for i in range(K):
+        if args.dump_outputs and i == K - 1:
+            wl.capture = True
+            last_start = counters.clone()
         step(i, kev[i])
     for w_ in pending:
         w_.wait()
@@ -765,6 +810,11 @@ def run_b200(args):
     e1.record()
     barrier()
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        # before the end-to-end and parity calls below, which reuse the buffers the last step wrote
+        outs = wl.outputs(torch)
+        outs["error_counters"] = (counters - last_start).cpu().numpy().astype(np.float64)
+        dump_outputs(args.dump_outputs, outs)
     ms_total = e0.elapsed_time(e1)
     kernel_ms = float(np.mean([a.elapsed_time(b) for a, b in kev]))
     t = torch.tensor([ms_total, kernel_ms], dtype=torch.float64, device="cuda")
@@ -892,6 +942,19 @@ def run_extras(torch):
     return out
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(path, arrays):
+    """--dump-outputs: DIR/<name>.npy per array, float32 / float64 only, at most 64 MB in all"""
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_LIMIT_BYTES, "outputs to dump take %d bytes" % total
+    os.makedirs(path, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 _JSON_FD = None
 
 
@@ -918,7 +981,13 @@ def main():
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--workload", default=DEFAULT_WORKLOAD, choices=sorted(WORKLOADS))
     ap.add_argument("--no-extras", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write what the last one computed to DIR/<name>.npy (B200 arm, rank 0)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the B200 arm")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
