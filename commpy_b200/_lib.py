@@ -6,9 +6,7 @@ import ctypes as C
 import os
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
-# COMMPY_B200_LIB (read once, at load time) points the binding at another build of the same C-ABI: used by the
-# kernel-variant experiments in scripts/ only
-LIB_PATH = os.environ.get("COMMPY_B200_LIB") or os.path.join(_HERE, "libcommpy_b200.so")
+LIB_PATH = os.path.join(_HERE, "libcommpy_b200.so")
 
 CPB_OK, CPB_EINVAL, CPB_EUNSUPPORTED, CPB_ECUDA, CPB_ENOMEM, CPB_ETRELLIS = range(6)
 CPB_U8, CPB_F32 = 0, 1

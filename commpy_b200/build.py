@@ -17,8 +17,7 @@ LIB = os.path.join(HERE, "libcommpy_b200.so")
 SOURCES = ["common.cu", "viterbi.cu", "bcjr.cu", "ldpc.cu", "demap.cu", "count.cu", "pipeline.cu", "hostapi.cu", "txlink.cu", "turbolink.cu"]
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
-         "-Xcompiler", "-fPIC", "--fmad=true",
-         "-DCPB_BUILDING=1"]
+         "-Xcompiler", "-fPIC", "--fmad=true"]
 
 
 def _newer(target, deps):

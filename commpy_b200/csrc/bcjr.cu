@@ -14,8 +14,8 @@
 //                            otherwise frame-major rows read as 16-byte vectors (map_decode).
 //   tpf::map_lin_kernel<T>   the same with per-step rescaling and separate prior / channel weights (non-systematic
 //                            compile-time trellises; cross-check of map_lin2 behind CPB_OPT_BCJR_PER_STEP_SCALING).
-//   tpf::map_ckpt_kernel /   log2-domain exact max* forms of the same thread mapping (unaligned lengths; compile-time
-//   tpf::map_tpf_kernel      switch CPB_BCJR_LOGDOMAIN).
+//   tpf::map_tpf_kernel<T>   log2-domain exact max* form of the same thread mapping, scalar loads, beta of every step in
+//                            global scratch (frame lengths not a multiple of 4, unaligned rows).
 //   map_kernel<S>            table-driven fallback for any other rate-1/2 trellis with <= 32 states: one LANE per state,
 //                            32/S frames per warp, neighbour metrics by warp shuffle, full-frame recursions (no windows),
 //                            log domain:
@@ -219,9 +219,14 @@ struct Params {
     const int32_t *rmap;
 };
 
-template <class T, int G>     // G = steps per vector access (4: float4 / uchar4, 1: scalar)
+// the log2-domain kernel for frame lengths that are not a multiple of 4 or rows that are not 16-byte aligned: scalar
+// loads, the beta of every step of the window in a global scratch
+template <class T>
 __global__ void __launch_bounds__(128) map_tpf_kernel(const Params p)
 {
+    // steps per group (one: scalar loads).  The one-step group loops are kept on purpose: written without them, the kernel
+    // compiles to a different instruction schedule from the one it has been tested and measured with.
+    constexpr int G = 1;
     constexpr int S = T::S;
     static_assert(T::valid(), "every state needs exactly two incoming edges");
     const int64_t g = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -239,14 +244,7 @@ __global__ void __launch_bounds__(128) map_tpf_kernel(const Params p)
         const float a = ys * p.c, b = yp * p.c;
         gm[0] = -a - b; gm[1] = b - a; gm[2] = a - b; gm[3] = a + b;      // output symbol (cs,cp): MSB = systematic
     };
-    auto load = [&](const float *q, int e0, float (&v)[G]) {            // elements e0 .. e0+G-1 (0-based)
-        if (G == 4) {
-            const float4 t = __ldg(reinterpret_cast<const float4 *>(q + e0));
-            v[0] = t.x; v[1 % G] = t.y; v[2 % G] = t.z; v[3 % G] = t.w;
-        } else {
-            v[0] = __ldg(q + e0);
-        }
-    };
+    auto load = [&](const float *q, int e0, float (&v)[G]) { v[0] = __ldg(q + e0); };
 
     // ---- backward: beta_t for t = tb .. lo+1, stored for t <= hi (inputs prefetched one group ahead)
     {
@@ -355,203 +353,16 @@ __global__ void __launch_bounds__(128) map_tpf_kernel(const Params p)
                 for (int s = 0; s < S; ++s) A[s] = An[s];
             }
             if (e0 >= lo) {
-                if (G == 4) {
-                    *reinterpret_cast<float4 *>(p.L_out + f * N + e0) = make_float4(Lv[0], Lv[1 % G], Lv[2 % G], Lv[3 % G]);
-                    if (p.bits_out) {
-                        uchar4 b;
-                        b.x = (p.mode == 1 && Lv[0] > 0.0f); b.y = (p.mode == 1 && Lv[1 % G] > 0.0f);
-                        b.z = (p.mode == 1 && Lv[2 % G] > 0.0f); b.w = (p.mode == 1 && Lv[3 % G] > 0.0f);
-                        *reinterpret_cast<uchar4 *>(p.bits_out + f * N + e0) = b;
-                    }
-                } else {
-                    p.L_out[f * N + e0] = Lv[0];
-                    if (p.bits_out) p.bits_out[f * N + e0] = (uint8_t)((p.mode == 1 && Lv[0] > 0.0f) ? 1 : 0);   // :148-152
-                }
+                p.L_out[f * N + e0] = Lv[0];
+                if (p.bits_out) p.bits_out[f * N + e0] = (uint8_t)((p.mode == 1 && Lv[0] > 0.0f) ? 1 : 0);   // :148-152
             }
         }
     }
 }
 
 // ------------------------------------------------------------------------------------------------
-// Checkpointed variant of the kernel above (the one that runs when N % 4 == 0): beta is written to HBM only every
-// CK-th step.  The forward sweep then works segment by segment: reload the CK steps of inputs into shared memory,
-// recompute the segment's beta backwards from its checkpoint (same operations in the same order as the first
-// sweep, so the same values), then run alpha / the a-posteriori LLRs forwards.  This trades +1 beta recursion per
-// step for 8x less beta traffic: the plain kernel moved 4.7 GB per pass for a batch of 8192 x 6144 (3.2 GB of it
-// beta), i.e. it was HBM bound on non-algorithmic bytes (profiles/r01_other_kernels_ncu.md).
-// Shared memory per thread: CK*(S+3) floats, thread-private columns [slot][thread] (conflict free).
-// ------------------------------------------------------------------------------------------------
-constexpr int CK = 8;
-
-template <class T>
-__global__ void __launch_bounds__(128) map_ckpt_kernel(const Params p)
-{
-    constexpr int S = T::S;
-    constexpr int G = 4;
-    extern __shared__ float smem_f[];
-    const int tid = threadIdx.x, bd = blockDim.x;
-    float *sb = smem_f;                         // [CK][S][bd]   beta of the current segment
-    float *si = smem_f + CK * S * bd;           // [CK][3][bd]   sys, par, La of the current segment
-    const int64_t g = (int64_t)blockIdx.x * bd + tid;
-    if (g >= p.NT) return;
-    const int w = (int)(g / p.bp);
-    const int64_t f = g - (int64_t)w * p.bp;
-    if (f >= p.batch) return;
-    const int N = p.N;
-    const int lo = w * p.win, hi = min(N, lo + p.win);
-    const float *fs = p.sys + f * N, *fp = p.par + f * N, *fl = p.La + f * N;
-    float *ck = p.beta + g;                     // checkpoints: [(j*S + s) * NT + thread], j = segment index
-
-    auto branch = [&](float ys, float yp, float (&gm)[4]) {
-        const float a = ys * p.c, b = yp * p.c;
-        gm[0] = -a - b; gm[1] = b - a; gm[2] = a - b; gm[3] = a + b;
-    };
-    auto beta_step = [&](float (&B)[S], float ys, float yp, float la_raw, int t) {     // beta_t -> beta_{t-1}
-        float gm[4];
-        branch(ys, yp, gm);
-        const float la = la_raw * LOG2E;
-        float Bn[S];
-#pragma unroll
-        for (int s = 0; s < S; ++s)
-            Bn[s] = maxstar2(B[T::ns(s, 0)] + gm[T::out(s, 0)], B[T::ns(s, 1)] + gm[T::out(s, 1)] + la);
-        if ((t & 3) == 1) {
-            float m = Bn[0];
-#pragma unroll
-            for (int s = 1; s < S; ++s) m = fmaxf(m, Bn[s]);
-#pragma unroll
-            for (int s = 0; s < S; ++s) Bn[s] -= m;
-        }
-#pragma unroll
-        for (int s = 0; s < S; ++s) B[s] = Bn[s];
-    };
-    auto ld4 = [&](const float *q, int e0, float (&v)[G]) {
-        const float4 t = __ldg(reinterpret_cast<const float4 *>(q + e0));
-        v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
-    };
-
-    // ---- backward sweep, checkpoint beta at the end of every segment
-    {
-        float B[S];
-        const int tb = min(N, hi + WARM);
-#pragma unroll
-        for (int s = 0; s < S; ++s) B[s] = 0.0f;
-        float ns_[G], np_[G], nl_[G];
-        ld4(fs, tb - G, ns_); ld4(fp, tb - G, np_); ld4(fl, tb - G, nl_);
-        for (int e1 = tb; e1 > lo; e1 -= G) {
-            float vs[G], vp[G], vl[G];
-#pragma unroll
-            for (int i = 0; i < G; ++i) { vs[i] = ns_[i]; vp[i] = np_[i]; vl[i] = nl_[i]; }
-            if (e1 - G > lo) { ld4(fs, e1 - 2 * G, ns_); ld4(fp, e1 - 2 * G, np_); ld4(fl, e1 - 2 * G, nl_); }
-#pragma unroll
-            for (int i = G - 1; i >= 0; --i) {
-                const int t = e1 - (G - 1 - i);
-                if (t <= hi && (((t - lo) % CK) == 0 || t == hi)) {
-                    const int j = (t - lo + CK - 1) / CK - 1;
-#pragma unroll
-                    for (int s = 0; s < S; ++s) ck[((int64_t)j * S + s) * p.NT] = B[s];
-                }
-                beta_step(B, vs[i], vp[i], vl[i], t);
-            }
-        }
-    }
-    // ---- forward sweep
-    float A[S];
-    const int ta = max(0, lo - WARM);
-#pragma unroll
-    for (int s = 0; s < S; ++s) A[s] = (ta == 0 && s != 0) ? NEGM : 0.0f;
-    auto alpha_step = [&](float ys, float yp, float la_raw, int t, const float *bt, bool emit, float &Lout) {
-        float gm[4];
-        branch(ys, yp, gm);
-        const float la = la_raw * LOG2E;
-        float tx[2 * S];
-#pragma unroll
-        for (int e = 0; e < 2 * S; ++e) tx[e] = A[e >> 1] + gm[T::out(e >> 1, e & 1)];
-        if (emit) {
-            float x0[S], x1[S];
-#pragma unroll
-            for (int s = 0; s < S; ++s) {
-                x0[s] = tx[2 * s] + bt[T::ns(s, 0) * bd];
-                x1[s] = tx[2 * s + 1] + bt[T::ns(s, 1) * bd];
-            }
-            float m0 = x0[0], m1 = x1[0];
-#pragma unroll
-            for (int s = 1; s < S; ++s) { m0 = fmaxf(m0, x0[s]); m1 = fmaxf(m1, x1[s]); }
-            float s0 = 0.0f, s1 = 0.0f;
-#pragma unroll
-            for (int s = 0; s < S; ++s) { s0 += ex2(x0[s] - m0); s1 += ex2(x1[s] - m1); }
-            Lout = la_raw + LN2 * ((m1 + lg2(s1)) - (m0 + lg2(s0)));
-        }
-        float An[S];
-#pragma unroll
-        for (int n = 0; n < S; ++n) {
-            const int ea = T::pred(n, 0), eb = T::pred(n, 1);
-            An[n] = maxstar2(tx[ea] + ((ea & 1) ? la : 0.0f), tx[eb] + ((eb & 1) ? la : 0.0f));
-        }
-        if ((t & 3) == 0) {
-            float m = An[0];
-#pragma unroll
-            for (int s = 1; s < S; ++s) m = fmaxf(m, An[s]);
-#pragma unroll
-            for (int s = 0; s < S; ++s) An[s] = fmaxf(An[s] - m, NEGM);
-        }
-#pragma unroll
-        for (int s = 0; s < S; ++s) A[s] = An[s];
-    };
-    // warm-up (no LLRs, no beta)
-    for (int e0 = ta; e0 < lo; e0 += G) {
-        float vs[G], vp[G], vl[G];
-        ld4(fs, e0, vs); ld4(fp, e0, vp); ld4(fl, e0, vl);
-        float dummy;
-#pragma unroll
-        for (int i = 0; i < G; ++i) alpha_step(vs[i], vp[i], vl[i], e0 + 1 + i, nullptr, false, dummy);
-    }
-    // segments
-    for (int s0 = lo, j = 0; s0 < hi; s0 += CK, ++j) {
-        const int ns = min(CK, hi - s0);                      // a multiple of 4
-        // inputs of the segment -> shared memory
-        for (int q = 0; q < ns; q += G) {
-            float vs[G], vp[G], vl[G];
-            ld4(fs, s0 + q, vs); ld4(fp, s0 + q, vp); ld4(fl, s0 + q, vl);
-#pragma unroll
-            for (int i = 0; i < G; ++i) {
-                si[((q + i) * 3 + 0) * bd + tid] = vs[i];
-                si[((q + i) * 3 + 1) * bd + tid] = vp[i];
-                si[((q + i) * 3 + 2) * bd + tid] = vl[i];
-            }
-        }
-        // beta of the segment, backwards from its checkpoint (beta at step s0+ns)
-        float B[S];
-#pragma unroll
-        for (int s = 0; s < S; ++s) B[s] = ck[((int64_t)j * S + s) * p.NT];
-        for (int i = ns - 1; i >= 0; --i) {
-#pragma unroll
-            for (int s = 0; s < S; ++s) sb[(i * S + s) * bd + tid] = B[s];          // beta_{s0+1+i}
-            beta_step(B, si[(i * 3 + 0) * bd + tid], si[(i * 3 + 1) * bd + tid], si[(i * 3 + 2) * bd + tid], s0 + 1 + i);
-        }
-        // alpha / LLR forwards
-        for (int q = 0; q < ns; q += G) {
-            float Lv[G];
-#pragma unroll
-            for (int i = 0; i < G; ++i) {
-                const int k = q + i;
-                alpha_step(si[(k * 3 + 0) * bd + tid], si[(k * 3 + 1) * bd + tid], si[(k * 3 + 2) * bd + tid], s0 + 1 + k,
-                           sb + (k * S) * bd + tid, true, Lv[i]);
-            }
-            const int e0 = s0 + q;
-            *reinterpret_cast<float4 *>(p.L_out + f * N + e0) = make_float4(Lv[0], Lv[1], Lv[2], Lv[3]);
-            if (p.bits_out) {
-                uchar4 b;
-                b.x = (p.mode == 1 && Lv[0] > 0.0f); b.y = (p.mode == 1 && Lv[1] > 0.0f);
-                b.z = (p.mode == 1 && Lv[2] > 0.0f); b.w = (p.mode == 1 && Lv[3] > 0.0f);
-                *reinterpret_cast<uchar4 *>(p.bits_out + f * N + e0) = b;
-            }
-        }
-    }
-}
-
-// ------------------------------------------------------------------------------------------------
-// Probability-domain variant (what actually runs for N % 4 == 0): the log-domain kernels above spend 66 MUFU
-// operations per trellis step (ex2 + lg2 per max*) and are bound by the 16-lane XU pipe.  The reference itself
+// Probability-domain variant (what actually runs for N % 4 == 0): the log-domain kernel above spends 66 MUFU
+// operations per trellis step (ex2 + lg2 per max*) and is bound by the 16-lane XU pipe.  The reference itself
 // works with probabilities renormalised every step (turbo.py:106-111, :155); doing the same in fp32 needs only
 // multiplies and adds for the recursions:
 //   branch weight of output symbol (cs, cp), relative to the best symbol of the step (all weights <= 1, no
@@ -560,9 +371,17 @@ __global__ void __launch_bounds__(128) map_ckpt_kernel(const Params p)
 //   beta_{t-1}(s) = sum_u p_u w(s,u) beta_t(ns(s,u)),  alpha_t(ns) += p_u w(s,u) alpha_{t-1}(s),  both rescaled to sum 1
 //   L_t = La + ln( sum_s alpha w(s,1) beta / sum_s alpha w(s,0) beta )
 // i.e. 2 + 1 ex2, 3 reciprocals and 2 lg2 per step instead of 66 MUFU ops.  |a|, |b|, |La log2e| are clamped to 60
-// so nothing reaches the fp32 exponent limits; the clamp only acts where |LLR| > ~80.  Beta is checkpointed every
-// CK steps and recomputed per segment in shared memory exactly like map_ckpt_kernel.
+// so nothing reaches the fp32 exponent limits; the clamp only acts where |LLR| > ~80.
+// Beta is written to HBM only every CK-th step.  The forward sweep then works segment by segment: reload the CK steps of
+// inputs into shared memory, recompute the segment's beta backwards from its checkpoint (same operations in the same
+// order as the first sweep, so the same values), then run alpha / the a-posteriori LLRs forwards.  This trades +1 beta
+// recursion per step for 8x less beta traffic: map_tpf_kernel, which stores the beta of every step, moved 4.7 GB per pass
+// for a batch of 8192 x 6144 (3.2 GB of it beta), i.e. it was HBM bound on non-algorithmic bytes
+// (profiles/r01_other_kernels_ncu.md).
+// Shared memory per thread: CK*(S+3) floats, thread-private columns [slot][thread] (conflict free).
 // ------------------------------------------------------------------------------------------------
+constexpr int CK = 8;
+
 __device__ __forceinline__ float rcp(float x) { float y; asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(y) : "f"(x)); return y; }
 
 template <class T>
@@ -773,17 +592,10 @@ __host__ __device__ constexpr bool systematic()
 }
 
 constexpr float RESCALE_FLOOR = 9.5367431640625e-07f;      // 2^-20
-#ifndef CPB_MAP_PFF
-#define CPB_MAP_PFF 1              // forward sweep: segments (of 8 steps, with their beta checkpoint) in flight per thread
-#endif
-constexpr int PFF = CPB_MAP_PFF;
-
-#ifndef CPB_MAP_MINB
-#define CPB_MAP_MINB 12            // __launch_bounds__ minimum CTAs (= warps) per SM of map_lin2_kernel: <= 168 registers, three
+constexpr int LIN2_MIN_CTAS = 12;  // __launch_bounds__ minimum CTAs (= warps) per SM of map_lin2_kernel: <= 168 registers, three
                                    // warps per scheduler; the 1,536 warps of a config-3 pass (8,192 x 6 windows) are one wave
-#endif
 template <class T, bool SM>      // SM: step-major arrays (Params::pitch / rmap)
-__global__ void __launch_bounds__(32, CPB_MAP_MINB) map_lin2_kernel(const Params p)
+__global__ void __launch_bounds__(32, LIN2_MIN_CTAS) map_lin2_kernel(const Params p)
 {
     constexpr int S = T::S;
     constexpr int G = 4;
@@ -1093,19 +905,17 @@ __global__ void __launch_bounds__(32, CPB_MAP_MINB) map_lin2_kernel(const Params
     }
     // the inputs and the beta checkpoint of a segment are fetched while the previous segment is being processed
     static_assert(CK == 2 * G, "segment = two vector groups");
-    float xin[SM ? 1 : PFF][2][3][G], xck[SM ? 1 : PFF][S];
-    auto fetch_segment = [&](int s0, int j, float (&xi)[2][3][G], float (&xc)[S]) {
+    float xin[2][3][G], xck[S];
+    auto fetch_segment = [&](int s0, int j) {
         const int ns = min(CK, hi - s0);
 #pragma unroll
         for (int h = 0; h < 2; ++h)
-            if (h * G < ns) ld3(s0 + h * G, xi[h][0], xi[h][1], xi[h][2]);
+            if (h * G < ns) ld3(s0 + h * G, xin[h][0], xin[h][1], xin[h][2]);
 #pragma unroll
-        for (int s = 0; s < S; ++s) xc[s] = (ck + (uint32_t)(j * S) * NT32)[(uint32_t)s * NT32];
+        for (int s = 0; s < S; ++s) xck[s] = (ck + (uint32_t)(j * S) * NT32)[(uint32_t)s * NT32];
     };
     if constexpr (!SM) {
-#pragma unroll
-        for (int k = 0; k < PFF; ++k)
-            if (lo + k * CK < hi) fetch_segment(lo + k * CK, k, xin[k], xck[k]);
+        if (lo < hi) fetch_segment(lo, 0);
     }
     for (int s0 = lo, j = 0; s0 < hi; s0 += CK, ++j) {
         const int ns = min(CK, hi - s0);                        // 4 or 8
@@ -1119,38 +929,27 @@ __global__ void __launch_bounds__(32, CPB_MAP_MINB) map_lin2_kernel(const Params
 #pragma unroll
                 for (int a = 0; a < 3; ++a)
 #pragma unroll
-                    for (int i = 0; i < G; ++i) xin[0][h][a][i] = q[(h * 12 + a * 4 + i) * bd];
+                    for (int i = 0; i < G; ++i) xin[h][a][i] = q[(h * 12 + a * 4 + i) * bd];
 #pragma unroll
-            for (int s = 0; s < S; ++s) xck[0][s] = q[(24 + s) * bd];
+            for (int s = 0; s < S; ++s) xck[s] = q[(24 + s) * bd];
         }
 #pragma unroll
         for (int h = 0; h < 2; ++h) {
             if (h * G < ns) {
 #pragma unroll
                 for (int i = 0; i < G; ++i) {
-                    sg[(h * G + i) * bd + tid] = weights(xin[0][h][0][i], xin[0][h][1][i], xin[0][h][2][i]);
-                    sl[(h * G + i) * bd + tid] = xin[0][h][2][i];
+                    sg[(h * G + i) * bd + tid] = weights(xin[h][0][i], xin[h][1][i], xin[h][2][i]);
+                    sl[(h * G + i) * bd + tid] = xin[h][2][i];
                 }
             }
         }
         float B[S];
 #pragma unroll
-        for (int s = 0; s < S; ++s) B[s] = xck[0][s];
+        for (int s = 0; s < S; ++s) B[s] = xck[s];
         if constexpr (SM) {
             if (s0 + CK < hi) issue_segment(s0 + CK, j + 1, rn);
         } else {
-#pragma unroll
-            for (int k = 0; k + 1 < PFF; ++k) {
-#pragma unroll
-                for (int h = 0; h < 2; ++h)
-#pragma unroll
-                    for (int a = 0; a < 3; ++a)
-#pragma unroll
-                        for (int i = 0; i < G; ++i) xin[k][h][a][i] = xin[k + 1][h][a][i];
-#pragma unroll
-                for (int s = 0; s < S; ++s) xck[k][s] = xck[k + 1][s];
-            }
-            if (s0 + PFF * CK < hi) fetch_segment(s0 + PFF * CK, j + PFF, xin[PFF - 1], xck[PFF - 1]);
+            if (s0 + CK < hi) fetch_segment(s0 + CK, j + 1);
         }
         // beta of the segment, backwards from its checkpoint, block by block (beta_{s0+1+k} -> sb[k])
         auto store_beta = [&](int k, const float (&Bv)[S]) {
@@ -1232,7 +1031,7 @@ __global__ void __launch_bounds__(32, CPB_MAP_MINB) map_lin2_kernel(const Params
     }
 }
 
-// compile-time trellises this kernel is instantiated for (packed from commpy_b200's Trellis tables)
+// compile-time trellises the register-resident kernels are instantiated for (packed from commpy_b200's Trellis tables)
 using RscK4 = CT<8, 0xedfc96369120ull, 0xc99cc99cu>;         // Trellis([3], [[1, 0o15]], [[0o13]], 'rsc')  (config C3)
 using RscK4Legacy = CT<8, 0xedf5b2a4d120ull, 0xcc9999ccu>;   // Trellis([3], [[1, 0o15]], 0o13, 'rsc')
 using RscK3Legacy = CT<4, 0x2d9090ull, 0x99ccu>;             // Trellis([2], [[1, 7]], 5, 'rsc')     (test_convcode.py:37)
@@ -1249,6 +1048,20 @@ static bool matches(const int32_t *next, const int32_t *out, int S)
     return true;
 }
 
+// calls fn(T()) with the compile-time trellis T whose tables are the host tables (next, out) and returns true; false when
+// no compile-time trellis matches
+template <class Fn>
+static bool with_ct(const int32_t *next, const int32_t *out, int S, Fn &&fn)
+{
+    if (matches<RscK4>(next, out, S)) fn(RscK4());
+    else if (matches<RscK4Legacy>(next, out, S)) fn(RscK4Legacy());
+    else if (matches<RscK3Legacy>(next, out, S)) fn(RscK3Legacy());
+    else if (matches<FfK3>(next, out, S)) fn(FfK3());
+    else if (matches<RscK3>(next, out, S)) fn(RscK3());
+    else return false;
+    return true;
+}
+
 // steps per window: 1024 unless cpb_set_option(CPB_OPT_BCJR_WINDOW, w) asks for shorter windows (a multiple of 8, >= 128):
 // more threads per frame for small batches at the price of more warm-up steps.  The split depends only on N and this
 // explicit option, never on the batch, so a frame decodes identically whatever it is batched with.
@@ -1261,41 +1074,51 @@ static int window_len()
 }
 static int nwindows(int N) { const int w = window_len(); return (N > w + w / 2) ? (int)ceil_div(N, w) : 1; }
 
+// the checkpointed kernels read 16-byte vectors of a row (vec: N % 4 == 0 and aligned pointers) and work in blocks of 4
+// steps (a window that is not a multiple of CK ends in a 4-step segment)
+static bool blocked(bool vec, int win) { return vec && win % 4 == 0; }
+
+// map_lin2_kernel is written for systematic trellises with 4 or 8 states ...
+template <class T>
+constexpr bool lin2_trellis = systematic<T>() && T::S % 4 == 0;
+
+// ... and runs on them unless per-step scaling is asked for.  It is the only kernel that reads step-major arrays, so the
+// turbo loop runs step-major exactly when it takes the trellis and the frame length (step_major_ok).
+template <class T>
+static bool lin2_ok(bool vec, int win)
+{
+    return lin2_trellis<T> && blocked(vec, win) && !option(CPB_OPT_BCJR_PER_STEP_SCALING);
+}
+
 template <class T>
 static int launch(const Params &p, bool vec, cudaStream_t st)
 {
-    unsigned grid = (unsigned)ceil_div(p.NT, 128);
-    if (vec && (p.win % 4) == 0) {          // (a window that is not a multiple of CK ends in a 4-step segment)
-        // one warp per CTA: 49,152 threads (C3: 8,192 frames x 6 windows) are 1,536 CTAs instead of 384, which
-        // spreads evenly over 148 SMs (measured 0.88 vs 0.91 ms per pass)
-        const int bd = 32;
-        grid = (unsigned)ceil_div(p.NT, bd);
-        const size_t smem = sizeof(float) * CK * (T::S + 3) * bd;
-#ifdef CPB_BCJR_LOGDOMAIN
-        { const int rc_ = ensure_dyn_smem(reinterpret_cast<const void *>(map_ckpt_kernel<T>), smem); if (rc_) return rc_; }
-        map_ckpt_kernel<T><<<grid, bd, smem, st>>>(p);
-#else
-        if constexpr (systematic<T>() && T::S % 4 == 0) {
-            // (the kernel indexes its checkpoints with 32-bit offsets: always true for the chunks chunk_frames() makes)
-            if (!option(CPB_OPT_BCJR_PER_STEP_SCALING) && p.NT * (int64_t)(ceil_div(p.win, CK) * T::S) < (1ll << 31)) {
-                // beta, weights and L_int of a segment; step-major: + the 32 staged floats of the next segment (the beta /
-                // weight area doubles as the input ring of the backward sweep)
-                const size_t smem2 = (size_t)bd * (CK * (T::S / 4 * sizeof(float4) + sizeof(float4) + sizeof(float)) +
-                                                   (p.pitch ? 32 * sizeof(float) : 0));
-                void (*kern)(const Params) = p.pitch ? map_lin2_kernel<T, true> : map_lin2_kernel<T, false>;
-                { const int rc_ = ensure_dyn_smem(reinterpret_cast<const void *>(kern), smem2, p.pitch != 0); if (rc_) return rc_; }
-                kern<<<grid, bd, smem2, st>>>(p);
-                CPB_LAUNCH_CHECK();
-                return CPB_OK;
-            }
+    // the checkpointed kernels run one warp per CTA: 49,152 threads (C3: 8,192 frames x 6 windows) are 1,536 CTAs instead
+    // of 384, which spreads evenly over 148 SMs (measured 0.88 vs 0.91 ms per pass)
+    const int bd = 32;
+    const unsigned grid = (unsigned)ceil_div(p.NT, bd);
+    if constexpr (lin2_trellis<T>) {
+        // (the kernel indexes its checkpoints with 32-bit offsets: always true for the chunks chunk_frames() makes)
+        if (lin2_ok<T>(vec, p.win) && p.NT * (int64_t)(ceil_div(p.win, CK) * T::S) < (1ll << 31)) {
+            // beta, weights and L_int of a segment; step-major: + the 32 staged floats of the next segment (the beta /
+            // weight area doubles as the input ring of the backward sweep)
+            const size_t smem2 = (size_t)bd * (CK * (T::S / 4 * sizeof(float4) + sizeof(float4) + sizeof(float)) +
+                                               (p.pitch ? 32 * sizeof(float) : 0));
+            void (*kern)(const Params) = p.pitch ? map_lin2_kernel<T, true> : map_lin2_kernel<T, false>;
+            { const int rc_ = ensure_dyn_smem(reinterpret_cast<const void *>(kern), smem2, p.pitch != 0); if (rc_) return rc_; }
+            kern<<<grid, bd, smem2, st>>>(p);
+            CPB_LAUNCH_CHECK();
+            return CPB_OK;
         }
-        if (p.pitch) return CPB_EINVAL;
+    }
+    if (p.pitch) return CPB_EINVAL;                  // step-major arrays: map_lin2_kernel only
+    if (blocked(vec, p.win)) {
+        const size_t smem = sizeof(float) * CK * (T::S + 3) * bd;
         { const int rc_ = ensure_dyn_smem(reinterpret_cast<const void *>(map_lin_kernel<T>), smem); if (rc_) return rc_; }
         map_lin_kernel<T><<<grid, bd, smem, st>>>(p);
-#endif
-    } else if (p.pitch) return CPB_EINVAL;
-    else if (vec) map_tpf_kernel<T, 4><<<grid, 128, 0, st>>>(p);
-    else map_tpf_kernel<T, 1><<<grid, 128, 0, st>>>(p);
+    } else {
+        map_tpf_kernel<T><<<(unsigned)ceil_div(p.NT, 128), 128, 0, st>>>(p);
+    }
     CPB_LAUNCH_CHECK();
     return CPB_OK;
 }
@@ -1476,28 +1299,22 @@ static int launch_map(const cpbTrellis *t, int S, const float *sys, const float 
 {
     const int32_t *hn = nullptr, *ho = nullptr;
     cpb_trellis_host_tables(t, &hn, &ho);
-    {
-        tpf::Params p{};
-        p.sys = sys; p.par = par; p.La = La; p.batch = batch; p.bp = ceil_div(batch, 32) * 32;
-        p.N = N; p.nwin = tpf::nwindows(N); p.win = (p.nwin == 1) ? N : tpf::window_len();
-        p.c = tpf::LOG2E / noise_var; p.mode = mode; p.beta = beta; p.NT = (int64_t)p.nwin * p.bp;
-        p.L_out = L_out; p.bits_out = bits;
-        const bool vec = (N % 4 == 0) && ((((uintptr_t)sys | (uintptr_t)par | (uintptr_t)La | (uintptr_t)L_out) & 15) == 0) &&
-                         (bits == nullptr || (((uintptr_t)bits) & 3) == 0);
-        p.ext = 0;
-        p.pitch = pitch; p.rmap = rmap;
-#ifndef CPB_BCJR_LOGDOMAIN
-        if (want_ext && vec && (p.win % 4) == 0) p.ext = 1;
-#endif
-        if (pitch && !(vec && (p.win % 4) == 0 && p.ext)) return CPB_EINVAL;      // step_major_ok() said otherwise
-        if (pitch && (int64_t)N * pitch >= (1ll << 31)) return CPB_EINVAL;              // 32-bit element offsets in the kernel
+    tpf::Params p{};
+    p.sys = sys; p.par = par; p.La = La; p.batch = batch; p.bp = ceil_div(batch, 32) * 32;
+    p.N = N; p.nwin = tpf::nwindows(N); p.win = (p.nwin == 1) ? N : tpf::window_len();
+    p.c = tpf::LOG2E / noise_var; p.mode = mode; p.beta = beta; p.NT = (int64_t)p.nwin * p.bp;
+    p.L_out = L_out; p.bits_out = bits;
+    const bool vec = (N % 4 == 0) && ((((uintptr_t)sys | (uintptr_t)par | (uintptr_t)La | (uintptr_t)L_out) & 15) == 0) &&
+                     (bits == nullptr || (((uintptr_t)bits) & 3) == 0);
+    p.ext = (want_ext && tpf::blocked(vec, p.win)) ? 1 : 0;
+    p.pitch = pitch; p.rmap = rmap;
+    if (pitch && (int64_t)N * pitch >= (1ll << 31)) return CPB_EINVAL;              // 32-bit element offsets in the kernel
+    int rc = CPB_OK;
+    if (tpf::with_ct(hn, ho, S, [&](auto ct) { rc = tpf::launch<decltype(ct)>(p, vec, st); })) {
         if (did_ext) *did_ext = p.ext;
-        if (tpf::matches<tpf::RscK4>(hn, ho, S)) return tpf::launch<tpf::RscK4>(p, vec, st);
-        if (tpf::matches<tpf::RscK4Legacy>(hn, ho, S)) return tpf::launch<tpf::RscK4Legacy>(p, vec, st);
-        if (tpf::matches<tpf::RscK3Legacy>(hn, ho, S)) return tpf::launch<tpf::RscK3Legacy>(p, vec, st);
-        if (tpf::matches<tpf::FfK3>(hn, ho, S)) return tpf::launch<tpf::FfK3>(p, vec, st);
-        if (tpf::matches<tpf::RscK3>(hn, ho, S)) return tpf::launch<tpf::RscK3>(p, vec, st);
+        return rc;
     }
+    if (pitch) return CPB_EINVAL;                    // step-major arrays: map_lin2_kernel only
     // any other rate-1/2 trellis with 2..32 states: table-driven lane-per-state kernel
     if (did_ext) *did_ext = 0;
     const int32_t *nx = cpb_trellis_next_dev(t), *ot = cpb_trellis_out_dev(t), *pd = cpb_trellis_pred_dev(t);
@@ -1525,24 +1342,18 @@ static int check_trellis(const cpbTrellis *t, int *S)
     return CPB_OK;
 }
 
-// the turbo loop runs on step-major arrays when the block-rescaled kernel takes the trellis and the frame length
+// the turbo loop runs on step-major arrays when the block-rescaled kernel takes the trellis and the frame length (the
+// arrays are the 16-byte aligned workspace; the kernel reads the interleaver as int4)
 static bool step_major_ok(const cpbTrellis *t, int S, int N, const int32_t *perm_dev)
 {
-#ifdef CPB_BCJR_LOGDOMAIN
-    return false;
-#else
-    if (option(CPB_OPT_BCJR_PER_STEP_SCALING) || option(CPB_OPT_TURBO_FRAME_MAJOR)) return false;
-    if (N % 4 != 0 || (reinterpret_cast<uintptr_t>(perm_dev) & 15) != 0) return false;
-    const int nwin = tpf::nwindows(N);
-    const int win = (nwin == 1) ? N : tpf::window_len();
-    if (win % 4 != 0) return false;
+    if (option(CPB_OPT_TURBO_FRAME_MAJOR)) return false;
+    const bool vec = (N % 4 == 0) && (reinterpret_cast<uintptr_t>(perm_dev) & 15) == 0;
+    const int win = (tpf::nwindows(N) == 1) ? N : tpf::window_len();
     const int32_t *hn = nullptr, *ho = nullptr;
     cpb_trellis_host_tables(t, &hn, &ho);
-    return (tpf::matches<tpf::RscK4>(hn, ho, S) && tpf::systematic<tpf::RscK4>()) ||
-           (tpf::matches<tpf::RscK4Legacy>(hn, ho, S) && tpf::systematic<tpf::RscK4Legacy>()) ||
-           (tpf::matches<tpf::RscK3Legacy>(hn, ho, S) && tpf::systematic<tpf::RscK3Legacy>()) ||
-           (tpf::matches<tpf::RscK3>(hn, ho, S) && tpf::systematic<tpf::RscK3>());
-#endif
+    bool ok = false;
+    tpf::with_ct(hn, ho, S, [&](auto ct) { ok = tpf::lin2_ok<decltype(ct)>(vec, win); });
+    return ok;
 }
 
 static int64_t chunk_frames(int64_t batch, int N, int S)

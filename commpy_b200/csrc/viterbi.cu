@@ -99,16 +99,9 @@ constexpr int BD = 32;             // one warp per CTA: every synchronisation be
 constexpr int QBITS = 17;          // soft / unquantized: |quantised value| <= 2^17 (22 metric bits: 27 * 2^17 < 2^22)
 constexpr int QMAX = 1 << QBITS;
 constexpr int DMAX = 46;           // deepest traceback the fast path takes
-#ifndef CPB_TASK_CAP
-#define CPB_TASK_CAP 384
-#endif
-constexpr int TASK_CAP = CPB_TASK_CAP;
-#ifndef CPB_VITERBI_TBB
-#define CPB_VITERBI_TBB 24         // windows per traceback block (multiple of B, <= 28)
-#endif
-#ifndef CPB_VITERBI_TBB_SOFT
-#define CPB_VITERBI_TBB_SOFT CPB_VITERBI_TBB    // the same for the one-frame-per-thread (float input) kernels
-#endif      // retired paths kept per block and warp; beyond that they are finished inline
+constexpr int TASK_CAP = 384;      // retired paths kept per block and warp; beyond that they are finished inline
+constexpr int TBB = 24;            // windows per traceback block (multiple of B, <= 28), hard and soft kernels alike
+static_assert(TBB % 8 == 0, "bit-packed output: whole output bytes per traceback block");
 
 struct Params {
     const void *coded;
@@ -429,43 +422,26 @@ __device__ __forceinline__ void tb_block_body(const Smem<PACK> sm, int ts, int t
 }
 
 // the traceback is a call in the hard kernel (its 64 packed keys stay in callee-saved registers) and inlined in the
-// register-capped soft kernel (CPB_TB_INLINE_SOFT)
+// register-capped soft kernel
 template <class CODE, int PACK>
 __device__ __noinline__ void tb_block_call(const Smem<PACK> sm, int ts, int te, int slot_last, int D, int L, int NJ,
                                            uint8_t *out0, uint8_t *out1, int valid_mask, int out_vec8, bool final)
 {
     tb_block_body<CODE, PACK>(sm, ts, te, slot_last, D, L, NJ, out0, out1, valid_mask, out_vec8, final);
 }
-#ifndef CPB_QD_HARD
-#define CPB_QD_HARD 4              // input prefetch distance of the hard kernel, in pairs of steps
-#endif
-#ifndef CPB_QD_SOFT
-#define CPB_QD_SOFT 2              // input prefetch distance of the soft kernels, in pairs of steps
-#endif
-#ifndef CPB_SOFT_MIN_CTAS
-#define CPB_SOFT_MIN_CTAS 8        // __launch_bounds__ minimum CTAs per SM of the soft kernels (12 -- a 168-register cap -- measured 2.7 % slower)
-#endif
-#ifndef CPB_TB_DEPHASE
-#define CPB_TB_DEPHASE 8           // windows in the first traceback block of the second warp of a scheduler (0: off)
-#endif
-#ifndef CPB_TB_INLINE_SOFT
-#define CPB_TB_INLINE_SOFT 1
-#endif
-#ifndef CPB_TB_INLINE_HARD
-#define CPB_TB_INLINE_HARD 0
-#endif
 template <class CODE, int PACK>
 __device__ __forceinline__ void tb_block(const Smem<PACK> sm, int ts, int te, int slot_last, int D, int L, int NJ,
                                          uint8_t *out0, uint8_t *out1, int valid_mask, int out_vec8, bool final)
 {
-#ifdef CPB_EXP_NO_TB          // experiment: add-compare-select only (wrong output)
-    if (!final) return;
-#endif
-    if ((PACK == 1 && CPB_TB_INLINE_SOFT) || (PACK == 2 && CPB_TB_INLINE_HARD))
+    if constexpr (PACK == 1)
         tb_block_body<CODE, PACK>(sm, ts, te, slot_last, D, L, NJ, out0, out1, valid_mask, out_vec8, final);
     else
         tb_block_call<CODE, PACK>(sm, ts, te, slot_last, D, L, NJ, out0, out1, valid_mask, out_vec8, final);
 }
+constexpr int QD_HARD = 4;         // input prefetch distance of the hard kernel, in pairs of steps
+constexpr int QD_SOFT = 2;         // input prefetch distance of the soft kernels, in pairs of steps
+constexpr int SOFT_MIN_CTAS = 8;   // __launch_bounds__ minimum CTAs per SM of the soft kernels (12 -- a 168-register cap -- measured 2.7 % slower)
+constexpr int TB_DEPHASE = 8;      // windows in the first traceback block of the second warp of a scheduler (0: off)
 
 template <class CODE, int PACK, int QD, int IOP>
 __device__ __forceinline__ void viterbi_fast_body(const Params &p)
@@ -641,13 +617,13 @@ __device__ __forceinline__ void viterbi_fast_body(const Params &p)
     const int ts0 = (p.D - 2) & ~3;              // first traceback block starts at this boundary (windows exist from D-1)
     int ts_cur = ts0;
     int next_te = ts_cur + p.TBB;
-    if (CPB_TB_DEPHASE) {
+    if (TB_DEPHASE) {
         // The traceback is latency bound, the add-compare-select loop pipe bound: two warps that share a scheduler
         // (hardware warp slots w and w+4) should not trace back at the same time, so the second one ends its first
         // traceback block half a period early.  (Scheduling only: the output does not depend on the block boundaries.)
         uint32_t wid;
         asm("mov.u32 %0, %%warpid;" : "=r"(wid));
-        if ((wid >> 2) & 1u) next_te = ts_cur + CPB_TB_DEPHASE;   // a multiple of 8: output stores stay 8-byte aligned
+        if ((wid >> 2) & 1u) next_te = ts_cur + TB_DEPHASE;   // a multiple of 8: output stores stay 8-byte aligned
     }
     int nslot = 0;                               // ring slot the next completed block goes to
 
@@ -752,16 +728,16 @@ __device__ __forceinline__ void viterbi_fast_body(const Params &p)
 
 // hard decision: two u16x2-packed frames per thread
 template <class CODE>
-__global__ void __launch_bounds__(BD) viterbi_fast_kernel_hard(const Params p) { viterbi_fast_body<CODE, 2, CPB_QD_HARD, 0>(p); }
+__global__ void __launch_bounds__(BD) viterbi_fast_kernel_hard(const Params p) { viterbi_fast_body<CODE, 2, QD_HARD, 0>(p); }
 // the same with bit-packed input and output (1 bit per coded / decoded bit, np.packbits order): 8x less HBM and PCIe traffic
 template <class CODE>
-__global__ void __launch_bounds__(BD) viterbi_fast_kernel_hard_packed(const Params p) { viterbi_fast_body<CODE, 2, CPB_QD_HARD, 1>(p); }
+__global__ void __launch_bounds__(BD) viterbi_fast_kernel_hard_packed(const Params p) { viterbi_fast_body<CODE, 2, QD_HARD, 1>(p); }
 // soft / unquantized: one frame per thread, 32-bit keys
 template <class CODE>
-__global__ void __launch_bounds__(BD, CPB_SOFT_MIN_CTAS) viterbi_fast_kernel_soft(const Params p) { viterbi_fast_body<CODE, 1, CPB_QD_SOFT, 0>(p); }
+__global__ void __launch_bounds__(BD, SOFT_MIN_CTAS) viterbi_fast_kernel_soft(const Params p) { viterbi_fast_body<CODE, 1, QD_SOFT, 0>(p); }
 // the same on punctured rows: depuncturing (convcode.py:777-804) happens in the load
 template <class CODE>
-__global__ void __launch_bounds__(BD, CPB_SOFT_MIN_CTAS) viterbi_fast_kernel_soft_punct(const Params p) { viterbi_fast_body<CODE, 1, CPB_QD_SOFT, 2>(p); }
+__global__ void __launch_bounds__(BD, SOFT_MIN_CTAS) viterbi_fast_kernel_soft_punct(const Params p) { viterbi_fast_body<CODE, 1, QD_SOFT, 2>(p); }
 
 // Per-frame power-of-two scale for float input: the largest |value| of the frame (after the +-500 clip in 'soft'
 // mode, convcode.py:718-719; including the -1 padding of 'unquantized', :729-732) maps to at most 2^QBITS.
@@ -797,17 +773,14 @@ __global__ void frame_scale_kernel(const float *__restrict__ x, int64_t n_in, in
     }
 }
 
-template <class CODE, int PACK, int IOP = 0>
+template <class CODE, int PACK, int IOP>
 static int launch(const Params &p, cudaStream_t st)
 {
     const size_t smem = smem_bytes(p.RB, p.TBB, PACK);
     void (*kern)(const Params) = (IOP == 1) ? viterbi_fast_kernel_hard_packed<CODE>
                                : (IOP == 2) ? viterbi_fast_kernel_soft_punct<CODE>
                                : (PACK == 2) ? viterbi_fast_kernel_hard<CODE> : viterbi_fast_kernel_soft<CODE>;
-#ifndef CPB_SOFT_MAX_CARVEOUT
-#define CPB_SOFT_MAX_CARVEOUT 0
-#endif
-    { const int rc_ = ensure_dyn_smem(reinterpret_cast<const void *>(kern), smem, PACK == 1 && CPB_SOFT_MAX_CARVEOUT); if (rc_) return rc_; }
+    { const int rc_ = ensure_dyn_smem(reinterpret_cast<const void *>(kern), smem); if (rc_) return rc_; }
     const int64_t grid = ceil_div(p.batch, (int64_t)BD * PACK);
     kern<<<(unsigned)grid, BD, smem, st>>>(p);
     CPB_LAUNCH_CHECK();
@@ -1054,30 +1027,44 @@ static size_t generic_chunk(const cpbTrellis *t, int64_t batch, int64_t T, int64
     return (size_t)((T + 1) * (int64_t)(t->S + 1) * chunk);
 }
 
-static int launch_fast(const cpbTrellis *t, const fast::Params &p, int pack, int packed_io, cudaStream_t st)
+template <int PACK, int IOP>
+static int launch_fast(const cpbTrellis *t, const fast::Params &p, cudaStream_t st)
 {
-    if (packed_io == 2) {
-        if (t->fast_id == 1) return fast::launch<Code133_171, 1, 2>(p, st);
-        if (t->fast_id == 2) return fast::launch<Code171_133, 1, 2>(p, st);
-        if (t->fast_id == 3) return fast::launch<Code5_43, 1, 2>(p, st);
-        return fast::launch<Code5_7, 1, 2>(p, st);
+    switch (t->fast_id) {
+    case 1: return fast::launch<Code133_171, PACK, IOP>(p, st);
+    case 2: return fast::launch<Code171_133, PACK, IOP>(p, st);
+    case 3: return fast::launch<Code5_43, PACK, IOP>(p, st);
+    default: return fast::launch<Code5_7, PACK, IOP>(p, st);
     }
-    if (packed_io) {
-        if (t->fast_id == 1) return fast::launch<Code133_171, 2, 1>(p, st);
-        if (t->fast_id == 2) return fast::launch<Code171_133, 2, 1>(p, st);
-        if (t->fast_id == 3) return fast::launch<Code5_43, 2, 1>(p, st);
-        return fast::launch<Code5_7, 2, 1>(p, st);
-    }
-    if (pack == 2) {
-        if (t->fast_id == 1) return fast::launch<Code133_171, 2>(p, st);
-        if (t->fast_id == 2) return fast::launch<Code171_133, 2>(p, st);
-        if (t->fast_id == 3) return fast::launch<Code5_43, 2>(p, st);
-        return fast::launch<Code5_7, 2>(p, st);
-    }
-    if (t->fast_id == 1) return fast::launch<Code133_171, 1>(p, st);
-    if (t->fast_id == 2) return fast::launch<Code171_133, 1>(p, st);
-    if (t->fast_id == 3) return fast::launch<Code5_43, 1>(p, st);
-    return fast::launch<Code5_7, 1>(p, st);
+}
+
+// the launch parameters every fast-path entry point sets alike; CPB_EUNSUPPORTED when the traceback ring does not fit in
+// shared memory
+static int fast_params(fast::Params &p, const void *coded, int64_t n_in, int64_t batch, int64_t L, int64_t T, int D,
+                       int mode, uint8_t *out)
+{
+    const int pack = (mode == CPB_VITERBI_HARD) ? 2 : 1;
+    p.coded = coded; p.n_in = n_in; p.batch = batch;
+    p.L = (int)L; p.T = (int)T; p.D = D;
+    p.TBB = fast::TBB;
+    p.NJ = (D > 8) ? (D - 8 + fast::B - 1) / fast::B : 0;
+    p.RB = p.NJ + p.TBB / fast::B;
+    p.mode = mode; p.out = out;
+    p.out_vec8 = ((L % 8) == 0 && (((uintptr_t)out) % 8) == 0) ? 1 : 0;
+    p.met_mask = (pack == 2) ? ~fast::KeyOps<2>::FMASK : ~fast::KeyOps<1>::FMASK;
+    return (fast::smem_bytes(p.RB, p.TBB, pack) > device_props().smem_optin) ? CPB_EUNSUPPORTED : CPB_OK;
+}
+
+// float input: the power-of-two scale of every frame (over the first n_used values of its row) into the workspace, past
+// its first 256 bytes
+static int frame_scales(fast::Params &p, const float *x, int64_t n_in, int64_t n_used, void *ws, cudaStream_t st)
+{
+    float *sc = reinterpret_cast<float *>(reinterpret_cast<unsigned char *>(ws) + 256);
+    p.frame_scale = sc;
+    const int wpb = 8;
+    fast::frame_scale_kernel<<<(unsigned)ceil_div(p.batch, wpb), wpb * 32, 0, st>>>(x, n_in, n_used, p.batch, p.mode, sc);
+    const cudaError_t e = cudaGetLastError();
+    return (e == cudaSuccess) ? CPB_OK : record_cuda_error(e, "frame_scale_kernel", __FILE__, __LINE__);
 }
 
 extern "C" {
@@ -1120,36 +1107,17 @@ int cpb_viterbi_decode(const cpbTrellis *t, const void *coded_dev, int in_dtype,
     // the reference returns uninitialised memory when no traceback window ever closes (T < D-1) or D < 2
     if (L <= 0 || D < 2 || T < D - 1 || T > (1 << 24)) return CPB_EINVAL;
     cudaStream_t st = (cudaStream_t)stream;
-    const DeviceProps &dp = device_props();
 
     if (use_fast(t, D, mode, in_dtype)) {
-        fast::Params p{};
-        p.coded = coded_dev; p.n_in = n_in; p.batch = batch;
-        p.L = (int)L; p.T = (int)T; p.D = D;
-        p.TBB = (mode == CPB_VITERBI_HARD) ? CPB_VITERBI_TBB : CPB_VITERBI_TBB_SOFT;
-        p.NJ = (D > 8) ? (D - 8 + fast::B - 1) / fast::B : 0;
-        p.RB = p.NJ + p.TBB / fast::B;
-        p.mode = mode; p.out = out_bits_dev;
-        p.out_vec8 = ((L % 8) == 0 && (((uintptr_t)out_bits_dev) % 8) == 0) ? 1 : 0;
-        const int pack = (mode == CPB_VITERBI_HARD) ? 2 : 1;
-        const size_t need = 256 + (pack == 1 ? (size_t)batch * sizeof(float) : 0);
+        const bool hard = (mode == CPB_VITERBI_HARD);
         Scratch ws;
-        int rc = ws.acquire(workspace_dev, workspace_bytes, need, st);
+        int rc = ws.acquire(workspace_dev, workspace_bytes, 256 + (hard ? 0 : (size_t)batch * sizeof(float)), st);
         if (rc) return rc;
-        if (fast::smem_bytes(p.RB, p.TBB, pack) > dp.smem_optin) { ws.release(); return CPB_EUNSUPPORTED; }
-        p.met_mask = (pack == 2) ? ~fast::KeyOps<2>::FMASK : ~fast::KeyOps<1>::FMASK;
-        if (pack == 2) p.in_aligned = ((n_in % 4) == 0 && (((uintptr_t)coded_dev) % 4) == 0) ? 1 : 0;
-        else p.in_aligned = ((n_in % 4) == 0 && (((uintptr_t)coded_dev) % 16) == 0) ? 1 : 0;
-        if (pack == 1) {
-            float *sc = reinterpret_cast<float *>(reinterpret_cast<unsigned char *>(ws.ptr) + 256);
-            p.frame_scale = sc;
-            const int wpb = 8;
-            fast::frame_scale_kernel<<<(unsigned)ceil_div(batch, wpb), wpb * 32, 0, st>>>(
-                reinterpret_cast<const float *>(coded_dev), n_in, 2 * L, batch, mode, sc);
-            cudaError_t e = cudaGetLastError();
-            if (e != cudaSuccess) { ws.release(); return record_cuda_error(e, "frame_scale_kernel", __FILE__, __LINE__); }
-        }
-        rc = launch_fast(t, p, pack, 0, st);
+        fast::Params p{};
+        rc = fast_params(p, coded_dev, n_in, batch, L, T, D, mode, out_bits_dev);
+        p.in_aligned = ((n_in % 4) == 0 && (((uintptr_t)coded_dev) % (hard ? 4 : 16)) == 0) ? 1 : 0;
+        if (!rc && !hard) rc = frame_scales(p, reinterpret_cast<const float *>(coded_dev), n_in, 2 * L, ws.ptr, st);
+        if (!rc) rc = hard ? launch_fast<2, 0>(t, p, st) : launch_fast<1, 0>(t, p, st);
         ws.release();
         return rc;
     }
@@ -1161,7 +1129,7 @@ int cpb_viterbi_decode(const cpbTrellis *t, const void *coded_dev, int in_dtype,
     int rc = ws.acquire(workspace_dev, workspace_bytes, need, st);
     if (rc) return rc;
     const size_t smem = sizeof(float) * ((size_t)2 * t->S + (1u << t->n)) * gen::BD;
-    if (smem > dp.smem_optin) { ws.release(); return CPB_EUNSUPPORTED; }
+    if (smem > device_props().smem_optin) { ws.release(); return CPB_EUNSUPPORTED; }
     { const int rc_ = ensure_dyn_smem(reinterpret_cast<const void *>(gen::viterbi_generic_kernel), smem); if (rc_) { ws.release(); return rc_; } }
     cudaError_t e = cudaSuccess;
     for (int64_t f0 = 0; f0 < batch; f0 += stride) {
@@ -1192,23 +1160,14 @@ int cpb_viterbi_decode_packed(const cpbTrellis *t, const uint8_t *coded_packed_d
     cpb_viterbi_sizes(t, n_in, &L, &T);
     const int D = resolve_depth(t, L, tb_depth);
     if (L <= 0 || D < 2 || T < D - 1 || T > (1 << 24)) return CPB_EINVAL;
-    // whole bytes per row, whole output bytes per traceback block
-    if (!use_fast(t, D, CPB_VITERBI_HARD, CPB_U8) || (n_in % 8) != 0 || (L % 8) != 0 || ((D - 2) % 4) != 0 ||
-        (CPB_VITERBI_TBB % 8) != 0)
+    // whole bytes per row, whole output bytes per traceback block (fast::TBB % 8 == 0)
+    if (!use_fast(t, D, CPB_VITERBI_HARD, CPB_U8) || (n_in % 8) != 0 || (L % 8) != 0 || ((D - 2) % 4) != 0)
         return CPB_EUNSUPPORTED;
-    const DeviceProps &dp = device_props();
     fast::Params p{};
-    p.coded = coded_packed_dev; p.n_in = n_in; p.batch = batch;
-    p.L = (int)L; p.T = (int)T; p.D = D;
-    p.TBB = CPB_VITERBI_TBB;
-    p.NJ = (D > 8) ? (D - 8 + fast::B - 1) / fast::B : 0;
-    p.RB = p.NJ + p.TBB / fast::B;
-    p.mode = CPB_VITERBI_HARD; p.out = out_packed_dev;
+    const int rc = fast_params(p, coded_packed_dev, n_in, batch, L, T, D, CPB_VITERBI_HARD, out_packed_dev);
+    if (rc) return rc;
     p.out_vec8 = 2;
-    p.in_aligned = 0;
-    p.met_mask = ~fast::KeyOps<2>::FMASK;
-    if (fast::smem_bytes(p.RB, p.TBB, 2) > dp.smem_optin) return CPB_EUNSUPPORTED;
-    return launch_fast(t, p, 2, 1, (cudaStream_t)stream);
+    return launch_fast<2, 1>(t, p, (cudaStream_t)stream);
 }
 
 
@@ -1240,29 +1199,16 @@ int cpb_viterbi_decode_punctured(const cpbTrellis *t, const float *llr_punct_dev
     if (L <= 0 || D < 2 || T < D - 1 || T > (1 << 24)) return CPB_EINVAL;
     if (!use_fast(t, D, mode, CPB_F32)) return CPB_EUNSUPPORTED;
     cudaStream_t st = (cudaStream_t)stream;
-    const DeviceProps &dp = device_props();
     fast::Params p{};
-    p.coded = llr_punct_dev; p.n_in = n_depunct; p.batch = batch;
-    p.L = (int)L; p.T = (int)T; p.D = D;
-    p.TBB = CPB_VITERBI_TBB_SOFT;
-    p.NJ = (D > 8) ? (D - 8 + fast::B - 1) / fast::B : 0;
-    p.RB = p.NJ + p.TBB / fast::B;
-    p.mode = mode; p.out = out_bits_dev;
-    p.out_vec8 = ((L % 8) == 0 && (((uintptr_t)out_bits_dev) % 8) == 0) ? 1 : 0;
-    p.met_mask = ~fast::KeyOps<1>::FMASK;
-    p.punct_mask = mask; p.punct_len = punct_len; p.n_kept = n_kept;
-    if (fast::smem_bytes(p.RB, p.TBB, 1) > dp.smem_optin) return CPB_EUNSUPPORTED;
-    Scratch ws;
-    int rc = ws.acquire(workspace_dev, workspace_bytes, 256 + (size_t)batch * sizeof(float), st);
+    int rc = fast_params(p, llr_punct_dev, n_depunct, batch, L, T, D, mode, out_bits_dev);
     if (rc) return rc;
-    float *sc = reinterpret_cast<float *>(reinterpret_cast<unsigned char *>(ws.ptr) + 256);
-    p.frame_scale = sc;
-    const int wpb = 8;
+    p.punct_mask = mask; p.punct_len = punct_len; p.n_kept = n_kept;
+    Scratch ws;
+    rc = ws.acquire(workspace_dev, workspace_bytes, 256 + (size_t)batch * sizeof(float), st);
+    if (rc) return rc;
     // the erasures are zeros: the frame's scale is the largest magnitude among the values the depuncturing uses
-    fast::frame_scale_kernel<<<(unsigned)ceil_div(batch, wpb), wpb * 32, 0, st>>>(llr_punct_dev, n_kept, need, batch, mode, sc);
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) { ws.release(); return record_cuda_error(e, "frame_scale_kernel", __FILE__, __LINE__); }
-    rc = launch_fast(t, p, 1, 2, st);
+    rc = frame_scales(p, llr_punct_dev, n_kept, need, ws.ptr, st);
+    if (!rc) rc = launch_fast<1, 2>(t, p, st);
     ws.release();
     return rc;
 }

@@ -24,4 +24,4 @@ for _ in range(reps):
     viterbi_decode_batch(xt, tr, None, mode, out=out)
 e1.record(); torch.cuda.synchronize()
 ms = e0.elapsed_time(e1) / reps
-print("%s %s N=%d batch=%d: %.4f ms  %.3e cw/s" % (os.environ.get("COMMPY_B200_LIB", "default").split("_")[-1], mode, nbits, batch, ms, batch / ms * 1e3), flush=True)
+print("%s N=%d batch=%d: %.4f ms  %.3e cw/s" % (mode, nbits, batch, ms, batch / ms * 1e3), flush=True)

@@ -16,7 +16,6 @@ def timeit(fn, reps=3, warm=2):
     e1.record(); torch.cuda.synchronize()
     return e0.elapsed_time(e1) / reps
 
-tag = os.path.basename(os.environ.get("COMMPY_B200_LIB", "default"))
 rsc = helpers.rsc_k4(); N = 6144; il = RandInterlv(N, 1)
 s2 = 1.0 / (2 * (1 / 3) * 10 ** (1.0 / 10))
 modes = [("per-step, frame-major", 1, 1), ("block, frame-major", 0, 1), ("block, step-major", 0, 0)]
@@ -34,7 +33,7 @@ for batch, wins in ((8192, (0,)), (1024, (128,))):
             ms = timeit(lambda: turbo_decode_batch(y[0], y[1], y[2], rsc, s2, 6, il), reps=3, warm=1)
             out = turbo_decode_batch(y[0], y[1], y[2], rsc, s2, 6, il)
             if ref is None: ref = out.clone()
-            print("%-24s batch %5d window %4d %-22s: turbo 6 it %.3f ms = %.3e cw/s, bits differing from the first row %d of %d" % (
-                tag, batch, win or 1024, name, ms, batch / ms * 1e3, int((out != ref).sum()), out.numel()), flush=True)
+            print("batch %5d window %4d %-22s: turbo 6 it %.3f ms = %.3e cw/s, bits differing from the first row %d of %d" % (
+                batch, win or 1024, name, ms, batch / ms * 1e3, int((out != ref).sum()), out.numel()), flush=True)
 for o in (_lib.OPT_BCJR_WINDOW, _lib.OPT_BCJR_PER_STEP_SCALING, _lib.OPT_TURBO_FRAME_MAJOR):
     _lib.set_option(o, 0)
